@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 5 --warmup 3                    # CUDA path (this repo), workload C2
     python bench.py --config c3                                      # other BASELINE.json configs: c1, c3, c4
     python bench.py --impl reference --steps 3 --warmup 1            # the reference algorithm on the host cores (CPU oracle port)
+    python bench.py --dump-outputs /tmp/out                          # + the outputs of the last timed step as /tmp/out/<name>.npy
 
 Workloads (BASELINE.json `configs`; shapes from the reference's YAML files, see SURVEY.md section 8):
   c2 (default, the configuration `metric` is quoted on): one STEP = the hot-path work of one Replica-config frame:
@@ -82,6 +83,31 @@ def workload_config(name, points):
         mix.update({'map_iters': c['map'][0], 'map_rays': c['map'][1], 'geometry_stage_iters': g})
     w += f", S={c['S']}, {points} pts, 640x480"
     return {'workload': w, 'points': points, 'iteration_mix': mix, 'parallelism': 'scene-per-gpu'}
+
+
+DUMP_ROWS = 1 << 16          # --dump-outputs: a longer output is stored as a fixed seeded sample of this many rows
+DUMP_LIMIT = 64 << 20        # bytes of all dumped arrays together
+
+
+def sample_rows(t, seed=0):
+    """t, or a fixed seeded sample of DUMP_ROWS of its rows (kept in row order) when it has more."""
+    if t.shape[0] <= DUMP_ROWS:
+        return t
+    sel = np.sort(np.random.default_rng(seed).choice(t.shape[0], DUMP_ROWS, replace=False))
+    return t[torch.from_numpy(sel).to(t.device)]
+
+
+def dump_outputs(path, arrays):
+    """One path/<name>.npy per array: float64 arrays and integer ones (row indices) as float64, everything else as float32."""
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        host[name] = a.astype(np.float64 if a.dtype == np.float64 or np.issubdtype(a.dtype, np.integer) else np.float32)
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_LIMIT, f'--dump-outputs: {total} bytes, more than {DUMP_LIMIT}'
+    os.makedirs(path, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(path, f'{name}.npy'), a)
 
 
 def load_decoder_state():
@@ -300,6 +326,7 @@ class GpuScene:
                     self.mapper._iter('geometry' if it < g else 'color')
                 loss = self.mapper.loss
             rows = self.mapper.write_back()
+            self.last_n0, self.last_rows = n0, rows
             if self.share_map:
                 self.share_delta(n0, rows)
             samples += m_it * (m_rays // (1 + N_KEYFRAMES)) * (1 + N_KEYFRAMES) * self.S
@@ -310,6 +337,18 @@ class GpuScene:
 
     def captures(self):
         return self.tracker.captures + (self.mapper.captures if self.mapper else 0)
+
+    def outputs(self):
+        """What the last step hands its caller: the frame's pose estimate and its last tracking loss; with mapping also the mapping
+        loss, the points the map update appended, the feature rows the mapper optimised (row indices + geometry and colour
+        features, a fixed sample of DUMP_ROWS rows) and the colour decoder's parameters."""
+        out = dict(pose=self.tracker.best_cam, tracking_loss=self.tracker.loss)
+        if self.mapper is not None:
+            rows = sample_rows(self.last_rows)
+            out.update(mapping_loss=self.mapper.loss, added_points=self.npc.cloud_pos_tensor()[self.last_n0:], feature_rows=rows,
+                       geo_feats=self.npc.get_geo_feats()[rows], col_feats=self.npc.get_col_feats()[rows],
+                       color_decoder=torch.cat([p.detach().reshape(-1) for p in self.decoders.color_decoder.parameters()]))
+        return out
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -355,6 +394,7 @@ class RenderScene:
                 self.npc, self.decoders, b['rays_d'], b['rays_o'], self.device, 'color', gt_depth=b['depth'],
                 npc_geo_feats=self.npc.get_geo_feats(), npc_col_feats=self.npc.get_col_feats(), cloud_pos=self.npc.cloud_pos_tensor(),
                 dynamic_r_query=b['r_query'], _zero_depth=(None, None))
+        self.last = dict(depth=depth, uncertainty=unc, color=color)
         if from_host:
             self.out_host[:, 0].copy_(depth, non_blocking=True); self.out_host[:, 1].copy_(unc, non_blocking=True)
             self.out_host[:, 2:].copy_(color, non_blocking=True)
@@ -362,6 +402,10 @@ class RenderScene:
 
     def captures(self):
         return 0
+
+    def outputs(self):
+        """Depth, uncertainty and colour of every ray of the last batch."""
+        return self.last
 
     def knn_stats(self):
         """Mean number of candidate points the kNN kernel stages per query (SURVEY.md section 8d asks for C-bar)."""
@@ -412,6 +456,15 @@ class RerenderScene:
 
     def captures(self):
         return 0
+
+    def outputs(self):
+        """The image metrics and, of every frame this rank rendered, depth and colour at a fixed sample of DUMP_ROWS pixels."""
+        m = self.metrics
+        out = dict(psnr=m['psnr'], depth_l1=m['depth_l1'])
+        for k, (d, c) in sorted(m['rendered'].items()):
+            out[f'depth_frame{k}'] = sample_rows(d.reshape(-1), seed=k)
+            out[f'color_frame{k}'] = sample_rows(c.reshape(-1, 3), seed=k)
+        return out
 
 
 class HostSampler:
@@ -523,6 +576,10 @@ def run_ours(args):
     recaptures = scene.captures() - cap0
     host_stalls = sampler.report() if sampler else None
     ms1 = torch.cuda.memory_stats(device)
+    if args.dump_outputs and rank == 0:
+        # the last step of the second timed pass (inputs from pinned host memory): it replays the frames of the first pass on the
+        # map that pass has grown; with --gpus N only rank 0's scene is written
+        dump_outputs(args.dump_outputs, scene.outputs())
     alloc_diag = {k: ms1.get(k, 0) - ms0.get(k, 0) for k in ('num_device_alloc', 'num_device_free', 'num_alloc_retries', 'num_sync_all_streams')}
     alloc_diag['reserved_GB'] = round(ms1.get('reserved_bytes.all.current', 0) / 1e9, 2)
     map_ms = None
@@ -861,7 +918,13 @@ def main():
     ap.add_argument('--points', type=int, default=0, help='override the cloud size of the configuration')
     ap.add_argument('--share-map', action='store_true', help='N > 1: one scene replicated on every GPU, rank 0 maps and broadcasts the map delta (NCCL) every step')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write what the last timed step computed as '
+                    'DIR/<name>.npy (float32 / float64, at most 64 MiB; the inputs are seeded, so two builds compare output for output). '
+                    'That step is the last of the second timed pass (inputs from pinned host memory), which replays the frames of the '
+                    'first pass on the map the first pass has grown; with --gpus N only rank 0 writes its scene')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs dumps the CUDA arm (--impl ours)')
     if args.steps is None:
         # one host hiccup inside the map update's sync window costs a whole step (~45 ms: see DESIGN.md section 5), so the default
         # averages over 20 frame steps (1 s of device time) instead of 5

@@ -1,5 +1,5 @@
 #!/bin/bash
-# One GPU session (gpurun --timeout 3600 -- 'TAG=r02 bash profiles/gpu_session.sh'): full GPU suite (writes parity_r02.json), smoke,
+# One GPU session (TAG=r02 bash profiles/gpu_session.sh, about an hour): full GPU suite (parity table to profiles/parity_<TAG>.json or $PSL_PARITY_JSON), smoke,
 # the bench lines of every config + the reference arm, the ncu launch list and a full ncu capture of the step kernels.  Everything
 # that must come back goes to gpurun_out/ (the .ncu-rep with sources is ~25 MB, under the 64 MiB merge limit).
 # A/B switches (environment): PSL_LIB=/path/to/other.so (another build of the same sources), PSL_GEO_MMA=0 (FFMA geometry kernels),
@@ -7,7 +7,7 @@
 # PSL_CLOCKS_MS=<ms|0> (clock sampler period).  The 2-GPU lines: profiles/gpu_session_n2.sh under `gpurun --gpus 2`.
 mkdir -p gpurun_out
 T=${TAG:-f1}
-export PSL_PARITY_TO_GPURUN_OUT=1
+export PSL_PARITY_JSON=${PSL_PARITY_JSON:-$PWD/profiles/parity_${T}.json}     # the session's parity table, beside parity_r02.json
 ( time timeout 1200 python -m pytest tests -m gpu -q --maxfail=8 -p no:cacheprovider -rxX ) > gpurun_out/${T}_tests.log 2>&1
 echo "tests exit $?"; grep -E "^(FAILED|ERROR)|passed|failed" gpurun_out/${T}_tests.log | tail -8
 ( time timeout 300 python -c "import __graft_entry__ as g; g.smoke()" ) > gpurun_out/${T}_smoke.log 2>&1; echo "smoke exit $?"; tail -2 gpurun_out/${T}_smoke.log

@@ -58,7 +58,7 @@ def replay_randint(draws, device=None):
 
 
 class Errors:
-    """Collects (case, quantity, achieved error, limit) rows; the GPU session writes them to profiles/parity_r02.json."""
+    """Collects (case, quantity, achieved error, limit) rows; the GPU session writes them to $PSL_PARITY_JSON (tests/conftest.py)."""
     rows = []
 
     @classmethod
@@ -91,10 +91,10 @@ class Errors:
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# running the reference's own callers (baseline/_ref, a git-ignored copy of the reference's src/ + configs/ made by
-# __graft_entry__.build()) on top of the drop-in modules: INTEGRATION.md section 1, executed
+# running the reference's own callers (oracle/_ref, a git-ignored copy of the reference's src/ + configs/ made by
+# __graft_entry__.build() where it finds the reference) on top of the drop-in modules: INTEGRATION.md section 1, executed
 # ---------------------------------------------------------------------------------------------------------------------
-REF_COPY = os.path.join(C.ROOT, 'baseline', '_ref')
+REF_COPY = os.path.join(C.ROOT, 'oracle', '_ref')
 
 
 def have_reference_copy():
@@ -103,7 +103,7 @@ def have_reference_copy():
 
 def install_module_swap():
     """Register the drop-in modules under the reference's module paths and import the reference's Tracker / Mapper from
-    baseline/_ref.  -> (Tracker class, Mapper class, reference `src.common` module, reference `src.Mapper` module)."""
+    oracle/_ref.  -> (Tracker class, Mapper class, reference `src.common` module, reference `src.Mapper` module)."""
     import sys
     import types
     import point_slam_b200.src as b
@@ -132,7 +132,7 @@ def install_module_swap():
         del sys.modules[k]
     if REF_COPY not in sys.path:
         sys.path.insert(0, REF_COPY)
-    import src                                                   # the reference package (baseline/_ref/src)
+    import src                                                   # the reference package (oracle/_ref/src)
     assert os.path.realpath(os.path.dirname(src.__file__)).startswith(os.path.realpath(REF_COPY))
     sys.modules['src.neural_point'] = b.neural_point             # the swap of INTEGRATION.md section 1
     sys.modules['src.conv_onet'] = b.conv_onet

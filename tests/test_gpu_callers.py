@@ -3,9 +3,9 @@ oracle/make_golden_callers.py from the unmodified `Tracker.optimize_cam_in_batch
 
   * the fused iteration shells (graphed.FusedTracker / FusedMapper -- what bench.py times) fed the same pixels,
   * the drop-in `Renderer.render_img`,
-  * and the reference's OWN Tracker / Mapper code (baseline/_ref, unmodified) running on top of the drop-in modules
+  * and the reference's OWN Tracker / Mapper code (oracle/_ref, unmodified) running on top of the drop-in modules
     (the module swap of INTEGRATION.md section 1), replaying the same pixel draws.
-Achieved errors go to profiles/parity_r02.json (tests/conftest.py writes it at session end)."""
+Achieved errors go to $PSL_PARITY_JSON when it is set (tests/conftest.py writes it at session end)."""
 import contextlib
 import io
 import types
@@ -230,12 +230,13 @@ def test_render_img_matches_reference(name):
 # ---------------------------------------------------------------------------------------------------------------------
 # the reference's own Tracker / Mapper code on the drop-in modules
 # ---------------------------------------------------------------------------------------------------------------------
-need_ref = pytest.mark.skipif(not K.have_reference_copy(), reason='baseline/_ref missing: run __graft_entry__.build() where /root/reference exists')
+need_ref = pytest.mark.skipif(not K.have_reference_copy(),
+                              reason='oracle/_ref missing: __graft_entry__.build() copies the reference sources there where it finds them')
 
 
 @need_ref
 def test_reference_tracker_runs_on_the_drop_in():
-    """Unmodified src/Tracker.py:optimize_cam_in_batch (baseline/_ref) + drop-in NeuralPointCloud / POINT / Renderer on the B200,
+    """Unmodified src/Tracker.py:optimize_cam_in_batch (oracle/_ref) + drop-in NeuralPointCloud / POINT / Renderer on the B200,
     same pixels as the golden run -> same losses, pose gradients and poses as the unmodified reference on the CPU."""
     Tracker, _, ref_common, _ = K.install_module_swap()
     g = K.load('caller_tracker')
@@ -274,7 +275,7 @@ def test_reference_tracker_runs_on_the_drop_in():
 
 @need_ref
 def test_reference_mapper_runs_on_the_drop_in():
-    """Unmodified src/Mapper.py:optimize_map (baseline/_ref): add_neural_points, get_mask_from_c2w (the reference's numpy / cv2
+    """Unmodified src/Mapper.py:optimize_map (oracle/_ref): add_neural_points, get_mask_from_c2w (the reference's numpy / cv2
     code on the drop-in's cloud_pos()), four joint iterations with the stage switch -- on the drop-in modules on the B200."""
     _, Mapper, ref_common, ref_mapper = K.install_module_swap()
     from point_slam_b200.default_config import make_cfg

@@ -21,7 +21,7 @@ _WORST = {}
 
 
 def _tol(name, got, o32, o64, floor=1e-4, param=False):
-    """Checks one quantity and records the achieved error (profiles/parity_r02.json, written by tests/conftest.py).  The ~50
+    """Checks one quantity and records the achieved error ($PSL_PARITY_JSON, written by tests/conftest.py).  The ~50
     decoder-parameter gradients of a case are recorded as ONE row (the worst), the other quantities one row each."""
     from tests.callers import Errors
     e_gpu = C.rel_err(got.detach().cpu(), o64)
