@@ -312,7 +312,7 @@ int psl_wgrad_tc(const psl_decode_cfg* cfg, const psl_decoder_params* params_hos
  *                       and can be replayed as a CUDA graph.
  * ------------------------------------------------------------------------- */
 /* pixel sampling -> rays.  pix (n_frames*per_frame) int64: index into the (H - 2*H0... ) window, row = pix / win_w + H0,
- * column = pix % win_w + W0 (common.get_sample_uv, common.py:77-89).  Pose: `cam` (7) = [quaternion w,x,y,z (not normalised), T]
+ * column = pix % win_w + W0 (common.get_sample_uv, common.py:77-89); pix < 0 = no pixel: sampled depth 0 (zero loss weight).  Pose: `cam` (7) = [quaternion w,x,y,z (not normalised), T]
  * (common.get_camera_from_tensor, common.py:225-267) for ONE frame, or `c2w` (n_frames,3,4).  Outputs: rays_o/rays_d
  * (common.get_rays_from_uv, common.py:40-56), the sampled depth / colour and r2 = dyn_radius^2 (float64, may be NULL). */
 int psl_sample_rays(const int64_t* pix, int32_t n_frames, int32_t per_frame, int32_t H, int32_t W, int32_t H0, int32_t W0,
@@ -382,6 +382,31 @@ size_t psl_frustum_select_ws_bytes(int64_t n);
 int psl_frustum_select(const float* cloud_pos, int64_t n, const double* w2c_host, double fx, double fy, double cx, double cy,
                        const float* depth, int32_t H, int32_t W, int32_t edge, uint8_t* mask, int64_t* indices,
                        int32_t* count, void* ws, size_t ws_bytes, psl_stream_t stream);
+
+/* ------------------------------------------------------------------------- *
+ * per-frame colour gradient: dynamic-radius maps and gradient-based pixel selection
+ * ------------------------------------------------------------------------- */
+/* color (H,W,3) float32 -> float64 (H,W) maps, exactly as synth.sobel_radius_map computes them (Tracker.py:237-248):
+ * grey = 0.2125 R + 0.7154 G + 0.0721 B, 3x3 Sobel with [1,2,1]/4 smoothing and a zeroed 1-pixel border,
+ * mag = sqrt(gx^2 + gy^2) (not clipped), r_add = np.interp(clip(mag, 0, thr), [0, 0.01, thr], [r_add_max, r_add_max, r_add_min]),
+ * r_query = radius_query_ratio * r_add.  Any output may be NULL.  color_grad_threshold must exceed 0.01. */
+int psl_frame_grad(const float* color, int32_t H, int32_t W, double r_add_max, double r_add_min, double radius_query_ratio,
+                   double color_grad_threshold, double* mag, double* r_add, double* r_query, psl_stream_t stream);
+/* Candidate pixels of get_selected_index_with_grad (common.py:92-159): the k pixels of largest mag (H,W) over the whole image
+ * (ties: the smaller flat index first), of those the ones with H0 <= row < H1, W0 <= column < W1 and 0 < depth <= depth_max
+ * (+inf: no upper bound).  cand (room for k) receives their flat indices row * W + column in ascending order, *count (device
+ * int32) their number.  No host synchronisation.  ws: psl_grad_candidates_ws_bytes(H * W). */
+size_t psl_grad_candidates_ws_bytes(int32_t n_pixels);
+int psl_grad_candidates(const double* mag, const float* depth, int32_t H, int32_t W, int32_t H0, int32_t H1, int32_t W0, int32_t W1,
+                        float depth_max, int32_t k, int64_t* cand, int32_t* count, void* ws, size_t ws_bytes, psl_stream_t stream);
+/* n distinct entries of cand[0 .. *count) drawn uniformly without replacement: keys (capacity) uint32 are the caller's random
+ * keys, one per candidate slot; the n slots of smallest key (ties: smaller slot) are taken.  pix (n) int64 receives them as
+ * window-relative indices (row - H0) * win_w + (column - W0), the form psl_sample_rays / psl_pose_bwd take; when *count < n
+ * the slots beyond it are -1 ("no pixel": psl_sample_rays gives such a sample depth 0, so it carries no loss).  Shapes depend
+ * on capacity and n only.  ws: psl_pick_candidates_ws_bytes(capacity). */
+size_t psl_pick_candidates_ws_bytes(int32_t capacity);
+int psl_pick_candidates(const int64_t* cand, const int32_t* count, int32_t capacity, const uint32_t* keys, int32_t n, int32_t W,
+                        int32_t H0, int32_t W0, int32_t win_w, int64_t* pix, void* ws, size_t ws_bytes, psl_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_HERE)
 # PSL_LIB: load another build of the same sources (A/B experiments, e.g. one compiled with -DPSL_PRECISE_TRIG)
 LIB_PATH = os.environ.get('PSL_LIB') or os.path.join(_HERE, 'libpointslam_b200.so')
-SOURCES = ['psl_api.cu', 'psl_grid.cu', 'psl_decode_fwd.cu', 'psl_decode_bwd.cu', 'psl_geo_mma.cu', 'psl_composite.cu', 'psl_color_tc.cu', 'psl_color_tc_w16.cu', 'psl_color_h2.cu', 'psl_color_bwd_h2.cu', 'psl_color_bwd_tc.cu', 'psl_color_bwd_tc_w16.cu', 'psl_wgrad_tc.cu', 'psl_shell.cu', 'psl_map.cu']
+SOURCES = ['psl_api.cu', 'psl_grid.cu', 'psl_decode_fwd.cu', 'psl_decode_bwd.cu', 'psl_geo_mma.cu', 'psl_composite.cu', 'psl_color_tc.cu', 'psl_color_tc_w16.cu', 'psl_color_h2.cu', 'psl_color_bwd_h2.cu', 'psl_color_bwd_tc.cu', 'psl_color_bwd_tc_w16.cu', 'psl_wgrad_tc.cu', 'psl_shell.cu', 'psl_map.cu', 'psl_frame.cu']
 HEADERS = ['psl_common.cuh', 'psl_decode.cuh', 'psl_grid.cuh', 'psl_tc.cuh', 'psl_tc_layout.cuh', 'psl_color_tc.cuh', 'psl_color_bwd_tc.cuh', 'psl_composite.cuh']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '--threads', '4']
@@ -118,6 +118,11 @@ _SIGS = {
     'psl_frustum_select_ws_bytes': (_sz, [_i64]),
     'psl_frustum_select': (C.c_int, [_vp, _i64, C.POINTER(_f64), _f64, _f64, _f64, _f64, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp,
                                      _sz, _vp]),
+    'psl_frame_grad': (C.c_int, [_vp, _i32, _i32, _f64, _f64, _f64, _f64, _vp, _vp, _vp, _vp]),
+    'psl_grad_candidates_ws_bytes': (_sz, [_i32]),
+    'psl_grad_candidates': (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _f32, _i32, _vp, _vp, _vp, _sz, _vp]),
+    'psl_pick_candidates_ws_bytes': (_sz, [_i32]),
+    'psl_pick_candidates': (C.c_int, [_vp, _vp, _i32, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
 }
 EXPORTS = sorted(_SIGS)
 

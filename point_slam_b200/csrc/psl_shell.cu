@@ -48,7 +48,9 @@ __global__ void k_sample_rays(SampleArgs a) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= a.K * a.per) return;
     const int k = t / a.per;
-    const long long p = a.pix[t];
+    const long long p_in = a.pix[t];
+    const bool none = p_in < 0;                        // no pixel (psl_pick_candidates with fewer candidates than samples)
+    const long long p = none ? 0 : p_in;
     const int jj = (int)(p / a.ww) + a.H0, ii = (int)(p % a.ww) + a.W0;
     float R[9], T[3];
     if (a.cam) {
@@ -70,7 +72,7 @@ __global__ void k_sample_rays(SampleArgs a) {
         a.rays_o[t * 3 + r] = T[r];
     }
     const size_t px = ((size_t)k * a.H + jj) * a.W + ii;
-    a.b_depth[t] = a.depth[px];
+    a.b_depth[t] = none ? 0.f : a.depth[px];          // depth 0: outside the depth gate, zero loss weight
     a.b_color[t * 3] = a.color[px * 3]; a.b_color[t * 3 + 1] = a.color[px * 3 + 1]; a.b_color[t * 3 + 2] = a.color[px * 3 + 2];
     if (a.r2) { const double r = a.dyn[px]; a.r2[t] = r * r; }
 }
@@ -346,7 +348,7 @@ __global__ void __launch_bounds__(1024, 1) k_pose_bwd(const long long* __restric
     __shared__ float acc[12];
     float G[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, gT[3] = {0.f, 0.f, 0.f};
     for (int t = threadIdx.x; t < n; t += blockDim.x) {
-        const long long p = pix[t];
+        const long long p = pix[t] < 0 ? 0 : pix[t];     // the ray psl_sample_rays made for "no pixel" (its gradient is zero)
         float d[3];
         pixel_dir((float)((int)(p % ww) + W0), (float)((int)(p / ww) + H0), fx, fy, cx, cy, d);
 #pragma unroll

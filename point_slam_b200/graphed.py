@@ -466,13 +466,28 @@ class FusedTracker:
     of ~17 library kernels (tracker_iteration_fused + psl_pose_adam).  The decoder is frozen while tracking, so its operand
     images are packed once per frame.  separate_LR: the quaternion steps with lr/5 (Tracker.py:291-299); `best_cam` is the
     pose of the iteration with the smallest loss, which is what the reference keeps (candidate_cam_tensor, :340-343).
-    selected (optional, per frame): pre-selected pixel indices for tracking.sample_with_color_grad (Tracker.py:117-129); the
-    per-iteration subset is then drawn on the device (with replacement, where the reference uses np.random.choice without)."""
+    sample_with_color_grad (tracking.sample_with_color_grad, Tracker.py:117-129): load_frame builds the frame's candidate set --
+    the grad_ratio * n_pixels pixels of largest colour gradient, kept if inside the edge window with depth > 0
+    (ops.grad_candidates) -- and every iteration draws its n_pixels distinct pixels from it (ops.pick_candidates, without
+    replacement like the reference's np.random.choice); `picked` holds the last draw.  The candidate buffer has a fixed
+    capacity, so one captured graph serves every frame.  Off: uniform pixels of the window (torch.randint, common.py:77-89)."""
 
-    def __init__(self, renderer, npc, decoders, intr, n_pixels, device, edge=(20, 20), lr=0.002, w_color=0.5, separate_lr=True):
+    def __init__(self, renderer, npc, decoders, intr, n_pixels, device, edge=(20, 20), lr=0.002, w_color=0.5, separate_lr=True,
+                 sample_with_color_grad=False, grad_ratio=ops.GRAD_RATIO):
         require_supported(npc.cfg, 'FusedTracker', tracker=True)
         self.r, self.npc, self.dec, self.intr, self.n, self.dev, self.edge, self.w = renderer, npc, decoders, intr, n_pixels, device, edge, w_color
         H, W = intr['H'], intr['W']
+        self.sample_with_color_grad = bool(sample_with_color_grad)
+        if self.sample_with_color_grad:
+            lib = L.load()
+            cap = ops.grad_capacity(n_pixels, H, W, grad_ratio)
+            self.grad_ratio = int(grad_ratio)
+            self.mag = torch.zeros(H, W, dtype=torch.float64, device=device)
+            self.cand = torch.zeros(cap, dtype=torch.int64, device=device)
+            self.cand_count = torch.zeros(1, dtype=torch.int32, device=device)
+            self.cand_ws = torch.empty(lib.psl_grad_candidates_ws_bytes(H * W), dtype=torch.uint8, device=device)
+            self.pick_ws = torch.empty(lib.psl_pick_candidates_ws_bytes(cap), dtype=torch.uint8, device=device)
+            self.picked = torch.zeros(n_pixels, dtype=torch.int64, device=device)
         self.color = torch.zeros(H, W, 3, device=device)
         self.depth = torch.zeros(H, W, device=device)
         self.dyn = torch.zeros(H, W, dtype=torch.float64, device=device)
@@ -488,10 +503,18 @@ class FusedTracker:
         self.key = None
         self.captures = 0
 
+    def _window(self):
+        H, W = self.intr['H'], self.intr['W']
+        return (self.edge[0], H - self.edge[0], self.edge[1], W - self.edge[1])
+
     def _iter(self):
+        pix = self.pix
+        if pix is None and self.sample_with_color_grad:
+            pix = ops.pick_candidates(self.cand, self.cand_count, self.n, self.intr['W'], window=self._window(), pix=self.picked,
+                                      ws=self.pick_ws)
         tracker_iteration_fused(self.r, self.npc, self.dec, self.cam, self.adam.grad, self.color, self.depth, self.dyn, self.intr,
                                 self.n, self.dev, self.npc.get_geo_feats(), self.npc.get_col_feats(), self.npc.cloud_pos_tensor(),
-                                self.edge, self.loss, self.w, pack=self.pack, prepacked=True, pix=self.pix)
+                                self.edge, self.loss, self.w, pack=self.pack, prepacked=True, pix=pix)
         a = self.adam
         L.check(L.load().psl_pose_adam(L.ptr(self.cam), L.ptr(a.grad), L.ptr(a.m), L.ptr(a.v), L.ptr(a.t),
                                        self.lr * (0.2 if self.separate_lr else 1.0), self.lr, a.betas[0], a.betas[1], a.eps,
@@ -500,6 +523,10 @@ class FusedTracker:
 
     def load_frame(self, color, depth, dyn, cam_init):
         self.color.copy_(color, non_blocking=True); self.depth.copy_(depth, non_blocking=True); self.dyn.copy_(dyn, non_blocking=True)
+        if self.sample_with_color_grad:                     # the frame's candidate set (Tracker.py:117-129), once per frame
+            ops.frame_grad(self.color, self.npc.cfg, maps=False, mag_out=self.mag)
+            ops.grad_candidates(self.mag, self.depth, self.n, self.grad_ratio, window=self._window(), cand=self.cand,
+                                count=self.cand_count, ws=self.cand_ws)
         self.cam.copy_(cam_init)
         self.adam.reset()
         self.best_loss.fill_(1e20)

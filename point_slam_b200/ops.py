@@ -953,3 +953,85 @@ def frustum_select(cloud_pos: torch.Tensor, c2w, depth: torch.Tensor, H, W, fx, 
                 'psl_frustum_select')
     k = int(count.item())                  # the one synchronisation: the caller sizes its optimisable slices with it
     return (idx[:k], mask.bool()) if return_mask else idx[:k]
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# per-frame colour gradient: dynamic-radius maps and gradient-based pixel selection (csrc/psl_frame.cu)
+# ------------------------------------------------------------------------------------------------------------------
+GRAD_RATIO = 15              # get_selected_index_with_grad(ratio=15), common.py:92 (DESIGN.md section 1, stated assumptions)
+
+
+def frame_grad(color: torch.Tensor, cfg, maps: bool = True, mag_out: Optional[torch.Tensor] = None):
+    """The dynamic-radius maps of Tracker.py:237-248 / Mapper.py:686-704 and the gradient magnitude they come from, on the device:
+    -> (r_add, r_query, mag), float64 (H,W) each, equal to synth.sobel_radius_map(color, ...) for the maps.  `cfg`: the
+    configuration (its `pointcloud` section: radius_add_max, radius_add_min, radius_query_ratio, color_grad_threshold).
+    maps=False computes mag only (r_add, r_query are None); mag_out: a float64 (H,W) tensor to write mag into."""
+    lib = L.load()
+    pc = cfg['pointcloud'] if 'pointcloud' in cfg else cfg
+    col = _f32c(color)
+    H, W = int(col.shape[0]), int(col.shape[1])
+    assert col.shape == (H, W, 3), 'color must be (H,W,3)'
+    kw = dict(dtype=torch.float64, device=col.device)
+    mag = mag_out if mag_out is not None else torch.empty(H, W, **kw)
+    assert mag.shape == (H, W) and mag.dtype == torch.float64
+    r_add = torch.empty(H, W, **kw) if maps else None
+    r_query = torch.empty(H, W, **kw) if maps else None
+    L.check(lib.psl_frame_grad(L.ptr(col), H, W, float(pc['radius_add_max']), float(pc['radius_add_min']),
+                               float(pc['radius_query_ratio']), float(pc['color_grad_threshold']), L.ptr(mag), L.ptr(r_add),
+                               L.ptr(r_query), L.stream()), 'psl_frame_grad')
+    return r_add, r_query, mag
+
+
+def grad_capacity(n: int, H: int, W: int, ratio: int = GRAD_RATIO) -> int:
+    """Length of the candidate list of get_selected_index_with_grad for n samples: ratio * n, at most the image."""
+    return min(int(ratio) * int(n), int(H) * int(W))
+
+
+def grad_candidates(mag: torch.Tensor, depth: torch.Tensor, n: int, ratio: int = GRAD_RATIO, window=None, depth_max=None,
+                    cand: Optional[torch.Tensor] = None, count: Optional[torch.Tensor] = None, ws: Optional[torch.Tensor] = None):
+    """get_selected_index_with_grad (common.py:92-159) on the device, no host synchronisation: of the ratio * n pixels of
+    largest `mag` over the whole image (ties: smaller flat index first), the ones inside window = (H0, H1, W0, W1) (default: the
+    whole image) with 0 < depth <= depth_max (None: no upper bound).  -> (cand, count): cand (grad_capacity) int64, its first
+    count[0] entries the ascending flat indices row * W + column; count (1,) int32 on the device.  cand / count / ws may be
+    passed in (fixed buffers of a captured caller)."""
+    lib = L.load()
+    H, W = int(mag.shape[0]), int(mag.shape[1])
+    dev = mag.device
+    assert mag.dtype == torch.float64 and mag.is_contiguous()
+    dep = _f32c(depth)
+    assert dep.shape == (H, W)
+    H0, H1, W0, W1 = window if window is not None else (0, H, 0, W)
+    k = grad_capacity(n, H, W, ratio)
+    cand = cand if cand is not None else torch.empty(k, dtype=torch.int64, device=dev)
+    count = count if count is not None else torch.empty(1, dtype=torch.int32, device=dev)
+    assert cand.numel() >= k and cand.dtype == torch.int64 and count.dtype == torch.int32
+    ws_bytes = lib.psl_grad_candidates_ws_bytes(H * W)
+    ws = ws if ws is not None else torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    assert ws.numel() >= ws_bytes
+    dmax = float('inf') if depth_max is None else float(depth_max)
+    L.check(lib.psl_grad_candidates(L.ptr(mag), L.ptr(dep), H, W, int(H0), int(H1), int(W0), int(W1), dmax, k, L.ptr(cand),
+                                    L.ptr(count), L.ptr(ws), ws.numel(), L.stream()), 'psl_grad_candidates')
+    return cand, count
+
+
+def pick_candidates(cand: torch.Tensor, count: torch.Tensor, n: int, W: int, window=None, generator=None,
+                    pix: Optional[torch.Tensor] = None, ws: Optional[torch.Tensor] = None):
+    """n distinct candidates out of cand[:count] drawn uniformly without replacement (random_select / np.random.choice with
+    replace=False after get_selected_index_with_grad), as the window-relative flat indices psl_sample_rays takes:
+    (row - H0) * (W1 - W0) + column - W0 for window = (H0, H1, W0, W1) (default: the whole image of width W).  Slots beyond
+    count[0] are -1.  Static shapes and no host synchronisation: safe inside a CUDA-graph capture (the keys come from
+    torch.randint on `generator`, default: the device's default generator)."""
+    lib = L.load()
+    cap = int(cand.numel())
+    dev = cand.device
+    assert 1 <= n <= cap, 'need 1 <= n <= the candidate capacity'
+    H0, _, W0, W1 = window if window is not None else (0, None, 0, W)
+    keys = torch.randint(2 ** 31 - 1, (cap,), dtype=torch.int32, device=dev, generator=generator)
+    pix = pix if pix is not None else torch.empty(n, dtype=torch.int64, device=dev)
+    assert pix.numel() == n and pix.dtype == torch.int64
+    ws_bytes = lib.psl_pick_candidates_ws_bytes(cap)
+    ws = ws if ws is not None else torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    assert ws.numel() >= ws_bytes
+    L.check(lib.psl_pick_candidates(L.ptr(cand), L.ptr(count), cap, L.ptr(keys), int(n), int(W), int(H0), int(W0), int(W1 - W0),
+                                    L.ptr(pix), L.ptr(ws), ws.numel(), L.stream()), 'psl_pick_candidates')
+    return pix

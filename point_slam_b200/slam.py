@@ -13,12 +13,14 @@ have run (same stream), which is what `update_para_from_mapping` achieves with c
         est_c2w = slam.process_frame(idx, color, depth, gt_c2w)
 
 What is kept from the callers (cited lines) and what is not:
+  * per frame: the dynamic radius maps from the colour gradient (`Tracker.py:237-248`, `Mapper.py:686-704`) and the gradient
+    magnitude behind them, in one device pass (ops.frame_grad, the values synth.sobel_radius_map computes on the host);
   * tracking: constant-speed initialisation (`Tracker.py:279-286`), separate learning rates and the smallest-loss candidate
-    (`:289-349`, inside graphed.FusedTracker), gt pose for idx <= 1 (`:275-276`);
-  * mapping: dynamic radius maps from the colour gradient (`Mapper.py:686-704`; host, numpy -- SURVEY.md section 2 row 4 keeps the
-    samplers on the host), `add_neural_points` on `pixels_adding` random pixels (+ `pixels_based_on_color_grad` more with the
-    small radius; the reference picks those by colour gradient, here they are random pixels), iteration count scaled by the
-    number of added locations (`:404-406`), frustum feature selection (`:345`), keyframe selection 'global' or 'overlap'
+    (`:289-349`, inside graphed.FusedTracker), gt pose for idx <= 1 (`:275-276`), `sample_with_color_grad`: pixels drawn
+    without replacement from the frame's gradient candidates (`:117-129`, `common.py:92-159`);
+  * mapping: `add_neural_points` on `pixels_adding` random pixels + `pixels_based_on_color_grad` pixels drawn from the
+    gradient candidates of the whole image with 0 < depth <= 5 m (ratio 15), added with the small radius, iteration count scaled
+    by the number of added locations (`:404-406`), frustum feature selection (`:345`), keyframe selection 'global' or 'overlap'
     (`:170-235`), geometry -> colour stage switch (`:420-423`), keyframe insertion every `keyframe_every` frames (`:741-751`);
   * not reproduced: BA, exposure latents, colour refinement at the end of the run, visualiser / wandb / checkpoints (the
     checkpoint writer is `src/utils/Logger.py`), lazy_start.
@@ -27,8 +29,11 @@ import numpy as np
 import torch
 
 from . import graphed as G
-from . import ops, synth
+from . import ops
 from .src import common
+
+
+MAPPER_DEPTH_LIMIT = 5.0      # depth bound of the mapper's gradient pixels (DESIGN.md section 1, stated assumptions)
 
 
 class PointSLAM:
@@ -43,7 +48,8 @@ class PointSLAM:
         self.iters = m['iters'] if mapping_iters is None else mapping_iters
         self.iters_first = m['iters_first'] if first_iters is None else first_iters
         self.tracker = G.FusedTracker(renderer, npc, decoders, intr, t['pixels'], device, edge=(t['ignore_edge_H'], t['ignore_edge_W']),
-                                      lr=t['lr'], w_color=t['w_color_loss'], separate_lr=t['separate_LR'])
+                                      lr=t['lr'], w_color=t['w_color_loss'], separate_lr=t['separate_LR'],
+                                      sample_with_color_grad=t.get('sample_with_color_grad', False))
         self.mapper = None                     # built on the first mapped frame (needs a non-empty cloud for its capacity buffers)
         self.keyframes = []                    # dicts: idx, color, depth, c2w (est), dyn_r_query
         self.est = {}                          # idx -> (4,4) float32 device pose
@@ -53,10 +59,16 @@ class PointSLAM:
 
     # ---- helpers ------------------------------------------------------------------------------------------------------------
     def _radius_maps(self, color):
-        pc = self.cfg['pointcloud']
-        r_add, r_query = synth.sobel_radius_map(color.detach().cpu().numpy(), pc['radius_add_max'], pc['radius_add_min'],
-                                                pc['radius_query_ratio'], pc['color_grad_threshold'])
-        return torch.from_numpy(r_add).to(self.dev), torch.from_numpy(r_query).to(self.dev)
+        """-> (r_add, r_query, mag) float64 (H,W) device maps of the frame (no host round trip)."""
+        return ops.frame_grad(color, self.cfg)
+
+    def _grad_pixels(self, mag, depth, n):
+        """get_samples_with_pixel_grad of the mapper (common.py:92-159): n distinct pixels (flat indices) of the gradient candidates
+        of the whole image with 0 < depth <= 5 m -- fewer when there are fewer candidates."""
+        I = self.intr
+        cand, count = ops.grad_candidates(mag, depth, n, ops.GRAD_RATIO, depth_max=MAPPER_DEPTH_LIMIT)
+        pix = ops.pick_candidates(cand, count, n, I['W'], generator=self.gen)
+        return pix[pix >= 0]
 
     def _cam_tensor(self, c2w):
         return common.get_tensor_from_camera(c2w.detach().cpu()).to(self.dev).float()
@@ -121,7 +133,7 @@ class PointSLAM:
                 out.append(kf)
         return out
 
-    def map(self, idx, color, depth, c2w, r_add, r_query):
+    def map(self, idx, color, depth, c2w, r_add, r_query, mag):
         I, m, npc = self.intr, self.m, self.npc
         init = idx == 0
         n_add = m['pixels_adding']
@@ -131,7 +143,10 @@ class PointSLAM:
         for n_pix, grad in ((n_add, False), (m.get('pixels_based_on_color_grad', 0), True)):
             if n_pix <= 0:
                 continue
-            pix = torch.randint(0, I['H'] * I['W'], (n_pix,), device=self.dev, generator=self.gen)
+            if grad:
+                pix = self._grad_pixels(mag, depth, n_pix)
+            else:
+                pix = torch.randint(0, I['H'] * I['W'], (n_pix,), device=self.dev, generator=self.gen)
             j, i = pix // I['W'], pix % I['W']
             ro, rd = common.get_rays_from_uv(i.float(), j.float(), c2w[:3, :4], I['fx'], I['fy'], I['cx'], I['cy'], self.dev)
             gd = depth[j, i]
@@ -168,12 +183,12 @@ class PointSLAM:
     def process_frame(self, idx, color, depth, gt_c2w):
         """-> estimated (4,4) camera-to-world pose of frame idx.  Order of the reference's hand-shake: frame 0 is mapped before
         anything is tracked; a frame is tracked, then (every `every_frame` frames) mapped with the tracked pose."""
-        r_add, r_query = self._radius_maps(color)
+        r_add, r_query, mag = self._radius_maps(color)
         c2w = self.track(idx, color, depth, r_query, gt_c2w)
         self.est[idx] = c2w
         info = dict(idx=idx, mapped=False)
         if idx == 0 or idx % self.every_frame == 0:
-            added, iters, loss = self.map(idx, color, depth, c2w, r_add, r_query)
+            added, iters, loss = self.map(idx, color, depth, c2w, r_add, r_query, mag)
             info.update(mapped=True, added=added, iters=iters, points=self.npc.pts_num())
         self.log.append(info)
         return c2w
